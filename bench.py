@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the alignment hot path (BASELINE.json metric: GCUPS and reads/s, device-timed).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--reads B] [--config 2] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--reads B] [--config 2] [--impl reference] [--dump-outputs DIR]
 
 Workload (N = 1): BASELINE config 2 — 10 kb synthetic chimeric ONT-like reads vs 20 plasmid-like
 contigs of 7-9 kb, `--double-strand --circular`, local mode, default CLI scoring.  A step is one
@@ -13,6 +13,9 @@ A cell update = one (contig-strand position, read base) pair; every DP fill is c
 For N > 1 (torchrun, one rank per GPU) every rank aligns its own B reads (weak scaling, no
 collective: reads are independent); the timed region is bracketed by barriers and the max over
 ranks is taken.
+
+--dump-outputs DIR writes the chains the last timed step of each pass returned (rank 0) as .npy files (see dump_results),
+so that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import ctypes as C
@@ -25,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 ALG_OPS_PER_CELL = 32            # SURVEY.md section 8d: INT32 ops per cell update
 ALG_BYTES_PER_CELL = 0.5         # SURVEY.md section 8d: the traceback stream, <= 0.5 B per cell update
@@ -191,6 +195,60 @@ def parity_check(al, kw, named, reads, truth, e2e_chains, n_check=4, pool=32):
             "how": "GPU align_batch with per-read subset_words vs oracle/ on the same subsets, every field and operation of every chain"}
 
 
+DUMP_BYTES = 64 << 20   # --dump-outputs: the size of all files together stays below this
+CHAIN_FIELDS = ("score", "xstart", "xend", "ystart", "yend", "xlen", "ylen", "start_contig_idx", "end_contig_idx", "length")
+
+
+def dump_results(lib, prefix_map, handle, out_dir, name, budget):
+    """Writes the chains of a results handle (what the results accessors of `prefix_map` hand a caller, as in
+    stitch_b200._lib.read_results) as float64 arrays, exact for the 32-bit fields:
+
+        <name>_reads.npy   (r, 2)  read index, number of chains
+        <name>_chains.npy  (c, 11) read index, then CHAIN_FIELDS
+        <name>_ops.npy     (o, 4)  row of the chain in <name>_chains.npy, kind, a, b
+
+    A full batch of long reads has more operations than `budget` bytes hold, so the files cover a fixed sample of the reads:
+    the reads in a fixed random order (seed 0) as long as their rows fit the budget, written in read order.  Two builds that
+    compute the same chains write the same files."""
+    import numpy as np
+    from stitch_b200._abi import StitchChain, StitchOp
+    fn = {k: getattr(lib, v) for k, v in prefix_map.items()}
+    n_reads = fn["n_reads"](handle)
+    n_ch, n_op = C.c_uint64(), C.c_uint64()
+    ch_ptr = fn["chains"](handle, C.byref(n_ch))
+    op_ptr = fn["ops"](handle, C.byref(n_op))
+    chains = np.ctypeslib.as_array(ch_ptr, (n_ch.value,)) if n_ch.value else np.zeros(0, np.dtype(StitchChain))
+    ops = np.ctypeslib.as_array(op_ptr, (n_op.value,)) if n_op.value else np.zeros(0, np.dtype(StitchOp))
+    first, count = C.c_uint64(), C.c_uint32()
+    spans = []
+    for r in range(n_reads):
+        fn["read"](handle, r, C.byref(first), C.byref(count))
+        spans.append((first.value, count.value))
+    pick, used = [], 0
+    for r in np.random.default_rng(0).permutation(n_reads):
+        f, c = spans[r]
+        cost = 8 * (2 + 11 * c + 4 * int(chains["n_ops"][f:f + c].sum()))
+        if used + cost > budget:
+            break
+        pick.append(int(r))
+        used += cost
+    pick.sort()
+    none = np.zeros(0, np.int64)
+    rows = np.concatenate([np.arange(spans[r][0], spans[r][0] + spans[r][1]) for r in pick] + [none])
+    sel = chains[rows]
+    op_rows = np.concatenate([np.arange(o, o + n, dtype=np.int64) for o, n in zip(sel["ops_offset"], sel["n_ops"])] + [none])
+    sel_ops = ops[op_rows]
+    out = {
+        "reads": np.array([(r, spans[r][1]) for r in pick], dtype=np.float64).reshape(-1, 2),
+        "chains": np.column_stack([np.repeat(pick, [spans[r][1] for r in pick])] + [sel[f] for f in CHAIN_FIELDS]).astype(np.float64).reshape(-1, 11),
+        "ops": np.column_stack([np.repeat(np.arange(len(sel)), sel["n_ops"]), sel_ops["kind"], sel_ops["a"], sel_ops["b"]]).astype(np.float64).reshape(-1, 4),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}_{k}.npy"), a)
+    return {"reads": len(pick), "of_reads": n_reads, "chains": len(sel), "ops": len(sel_ops)}
+
+
 def via_cli(args):
     """The product's own multi-GPU path: ONE `stitch-b200 align --gpus N` process (a reader thread, one worker thread and one
     device context per GPU pulling batches from a bounded queue, formatter threads, an ordered BAM writer), timed by wall
@@ -270,7 +328,13 @@ def main():
     ap.add_argument("--cli-batch", type=int, default=256)
     ap.add_argument("--cli-pool", type=int, default=1000, help="--via-cli: distinct synthetic reads (cycled to --reads records)")
     ap.add_argument("--cli-out", default="/dev/null", help="--via-cli: where the BAM stream goes (default /dev/null: 650 KB per 10 kb read)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the chains the last timed step of each pass returned to DIR/*.npy "
+                                                          f"(at most {DUMP_BYTES >> 20} MB in all, a seeded sample of the reads)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.via_cli or args.cpu_sweep or args.impl != "stitch_b200"):
+        ap.error("--dump-outputs writes what the GPU passes compute: not with --via-cli, --cpu-sweep or --impl reference")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -346,25 +410,29 @@ def main():
         acc += len(r)
     offs[len(reads)] = acc
 
-    def step_device():
+    kept = {"device": None, "e2e": None}   # the results of the last step of each pass (read back after the timed region)
+
+    def step_device(last=False):
         res = C.c_void_p()
         rc = lib.stitch_custom_batch_device(al._h, C.c_void_p(d_reads.data_ptr()), offs, len(reads), C.byref(res))
         if rc != 0:
             raise RuntimeError(al.last_error())
-        lib.stitch_free_results(res)
+        if last:   # (kept only then: held across steps, results slowed this pass by 0.7 % on a B200 at 1000 W)
+            kept["device"] = res
+        else:
+            lib.stitch_free_results(res)
         return al.stats()
 
     host_buf, host_offs = _abi.pack_reads(reads)   # e2e: host buffers in, chains out
-    kept = {"res": None}                            # the results of the latest e2e step (read back after the timed region)
 
-    def step_e2e():
+    def step_e2e(last=False):   # (every step's results live until the next step frees them)
         res = C.c_void_p()
         rc = lib.stitch_align_batch(al._h, host_buf, host_offs, len(reads), None, 0, C.byref(res))
         if rc != 0:
             raise RuntimeError(al.last_error())
-        if kept["res"] is not None:
-            lib.stitch_free_results(kept["res"])
-        kept["res"] = res
+        if kept["e2e"] is not None:
+            lib.stitch_free_results(kept["e2e"])
+        kept["e2e"] = res
         return al.stats()
 
     def barrier():
@@ -379,8 +447,8 @@ def main():
                "tile_columns": 0, "quiet_tile_columns": 0}
         barrier()
         t0 = time.perf_counter()
-        for _ in range(steps):
-            s = fn()
+        for k in range(steps):
+            s = fn(last=k == steps - 1)
             agg["cells"] += s.cells; agg["fill_ms"] += s.fill_ms; agg["tb_ms"] += s.traceback_ms
             agg["launches"] += s.kernel_launches; agg["h2d"] += s.h2d_bytes; agg["d2h"] += s.d2h_bytes
             agg["fills"] += s.fills; agg["tb_bytes"] += s.traceback_bytes
@@ -405,8 +473,10 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    dt, agg = timed(step_device, args.steps)
-    clocks = sampler.stop() if rank == 0 else None
+    try:
+        dt, agg = timed(step_device, args.steps)
+    finally:   # (no nvidia-smi process outlives a failed step)
+        clocks = sampler.stop() if rank == 0 else None
     # e2e: one warm-up, then the same number of steps
     if args.no_e2e:
         dt_e, agg_e = dt, dict(agg)
@@ -474,9 +544,13 @@ def main():
                              "ops_per_cell": ALG_OPS_PER_CELL,
                              "peak_source": "stitch_measure_int32_peak (add+max issue-rate microbenchmark, measured in this run)"},
         }
+        if args.dump_outputs:
+            passes = [p for p in ("device", "e2e") if kept[p] is not None]
+            line["dump_outputs"] = {p: dump_results(lib, _lib.PRODUCT_RESULTS, kept[p], args.dump_outputs, p, (DUMP_BYTES - 4096) // len(passes))
+                                    for p in passes}
         if not args.no_parity_check:
             try:
-                e2e_chains = _lib.read_results(lib, _lib.PRODUCT_RESULTS, kept["res"])
+                e2e_chains = _lib.read_results(lib, _lib.PRODUCT_RESULTS, kept["e2e"])
                 line["parity_check"] = parity_check(al, kw, named, reads, truth, e2e_chains)
             except Exception as e:
                 line["parity_check"] = {"reads": 0, "ok": False, "error": str(e)}
@@ -486,8 +560,9 @@ def main():
             except Exception as e:   # the baseline is reported, never required for the GPU number
                 line["cpu_baseline"] = {"value": None, "unit": "GCUPS", "cores": 0, "kind": "port", "sample": f"failed: {e}"}
         print(json.dumps(line))
-    if kept["res"] is not None:
-        lib.stitch_free_results(kept["res"])
+    for res in kept.values():
+        if res is not None:
+            lib.stitch_free_results(res)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
