@@ -15,6 +15,10 @@
 // process-wide counters of the quiet-tile path (tests assert that tiles were actually skipped)
 static unsigned long long g_quiet_tiles = 0, g_quiet_skipped = 0, g_quiet_mat = 0;
 extern "C" void emul_quiet_counters(unsigned long long *out) { out[0] = g_quiet_tiles; out[1] = g_quiet_skipped; out[2] = g_quiet_mat; }
+// process-wide counters of the path each fill took (tests assert which path ran): out[0] packed fills, out[1] wide fills,
+// out[2 + LB] packed fills that ran with LB length bits (LB = 0 .. 31)
+static unsigned long long g_path[2 + 32] = {0};
+extern "C" void emul_path_counters(unsigned long long *out) { for (int k = 0; k < 2 + 32; ++k) out[k] = g_path[k]; }
 
 namespace stitch {
 namespace host {
@@ -138,7 +142,7 @@ static void emul_column(const ColumnArgs &A) {
 struct EmulBackend : Backend {
     Aligner &al;
     uint32_t dump_seq = 0;
-    uint32_t K, WINDOW, PACKED, QUIET, QUIET_EDGE, QUIET_LAST, CONE_AUDIT, CONE;
+    uint32_t K, WINDOW, PACKED, QUIET, QUIET_EDGE, QUIET_LAST, CONE_AUDIT, CONE, LB_MIN;
     explicit EmulBackend(Aligner &a) : al(a) {
         K = std::max<uint32_t>(1, env_u32("EMUL_K", 7));          // checkpoint spacing (columns)
         WINDOW = std::max<uint32_t>(1, env_u32("EMUL_WINDOW", 6));  // columns at the end of the read filled by the wide path
@@ -148,6 +152,7 @@ struct EmulBackend : Backend {
         QUIET_LAST = env_u32("EMUL_QUIET_LAST", 1);                 // 0: the last tile of a contig (row m) is always computed
         CONE = env_u32("EMUL_CONE", 1);                             // 0: the walk re-fills whole contigs
         CONE_AUDIT = env_u32("EMUL_CONE_AUDIT", 0);                 // 1: audit the dependency cone of the unit re-fills (experiment)
+        LB_MIN = env_u32("EMUL_LB_MIN", 0);                         // packed fills take at least this many length bits (widened LB)
     }
     ~EmulBackend() {
         if (std::getenv("EMUL_UNIT_STATS")) std::fprintf(stderr, "[emul units] cone %llu full %llu\n", (unsigned long long)cone_units, (unsigned long long)full_units);
@@ -745,8 +750,10 @@ struct EmulBackend : Backend {
         alloc(job, L, F);
         uint32_t m_max = 0;
         for (const auto &e : L.ent) m_max = std::max(m_max, e.m);
-        const uint32_t LB = (allow_packed && PACKED) ? pk_plan(sc, n, m_max) : 0;
-        if (!LB) { fill_wide(job, L, 0, track_from, F); return 0; }
+        uint32_t LB = (allow_packed && PACKED) ? pk_plan(sc, n, m_max) : 0;
+        if (!LB) { ++g_path[1]; fill_wide(job, L, 0, track_from, F); return 0; }
+        LB = std::max(LB, LB_MIN);   // (cuda_backend.cu run_chunk: one LB per launch, the largest any job needs)
+        ++g_path[0]; ++g_path[2 + (LB & 31u)];
         fill_packed_bulk(job, L, LB, F);
         // the tail restarts at the last checkpoint before the first column that can hold a final y-suffix
         // tracker (dp_core.h: first_candidate_column); column n is always part of it
@@ -928,3 +935,13 @@ Backend *stitch_make_backend(Aligner &al, int) { return new EmulBackend(al); }
 
 }  // namespace host
 }  // namespace stitch
+
+// pk_plan (dp_packed.h) of the scoring the product derives from these options: the length bits of the packed path, 0 = the
+// wide path, -1 = options the product refuses
+extern "C" int32_t emul_pk_plan(const stitch_opts *o, uint32_t n, uint32_t m_max) {
+    try {
+        return (int32_t)stitch::pk_plan(stitch::host::make_opts(*o).sc, n, m_max);
+    } catch (const stitch::host::Error &) {
+        return -1;
+    }
+}

@@ -45,8 +45,25 @@ def lib(strip=8):
     e.emul_destroy.argtypes = [C.c_void_p]
     e.emul_last_error.restype = C.c_char_p
     e.emul_last_error.argtypes = [C.c_void_p]
+    e.emul_pk_plan.restype = C.c_int32
+    e.emul_pk_plan.argtypes = [C.POINTER(StitchOpts), C.c_uint32, C.c_uint32]
+    e.emul_path_counters.restype = None
+    e.emul_path_counters.argtypes = [C.POINTER(C.c_ulonglong)]
     _libs[strip] = e
     return e
+
+
+def pk_plan(opts: StitchOpts, n, m_max, strip=8):
+    """pk_plan (stitch_b200/csrc/dp_packed.h) of the scoring the product derives from `opts`: the packed path's length bits,
+    0 = the wide path, -1 = options the product refuses."""
+    return lib(strip).emul_pk_plan(C.byref(opts), n, m_max)
+
+
+def path_counters(strip=8):
+    """Fills the emulator has run so far in this process: {"packed": .., "wide": .., "lb": {LB: packed fills with LB}}."""
+    out = (C.c_ulonglong * 34)()
+    lib(strip).emul_path_counters(out)
+    return {"packed": out[0], "wide": out[1], "lb": {k: out[2 + k] for k in range(32) if out[2 + k]}}
 
 
 class EmulError(RuntimeError):
