@@ -234,9 +234,23 @@ struct CudaBackend : host::Backend {
         return n.colrec * sizeof(ColRec) + n.cell * (sizeof(LastCell) + sizeof(SnRec)) + n.ck * sizeof(CellState) + n.pck * 4 +
                n.cksum * sizeof(CkSum) + n.gcol * 4;
     }
+    // Operation buffer of a read (run-length ops of all its chains).  It starts at (n/2 + 4C + 64) per chain for up to 8
+    // chains and grows x4 per retry of its chunk (`grow`), up to a bound no chain can exceed: M/X/D records consume a column
+    // each (<= n), an x-jump follows an M/X move or sits at column n (<= n + C + 1), x-clips need a jump between them
+    // (<= jumps + 2), y-clips <= 2, and I runs alternate with the rest (<= the rest + 1): 6n + 4C + 13 per chain.
+    static uint64_t chain_ops_bound(uint32_t n, uint32_t C) { return 6ull * n + 4ull * C + 16; }
+    uint64_t ops_max_of(const host::Job &j) const {
+        const uint32_t C = (uint32_t)al.layouts.layouts[j.layout].ent.size();
+        return std::min<uint64_t>(chain_ops_bound(j.n, C) * (j.walk == host::WALK_ALL ? C : 1), 0xffffffffull);
+    }
+    uint64_t ops_cap_of(const host::Job &j, uint32_t grow) const {
+        const uint32_t C = (uint32_t)al.layouts.layouts[j.layout].ent.size();
+        const uint64_t per_chain = j.n / 2 + 4ull * C + 64;
+        return std::min<uint64_t>((per_chain * (j.walk == host::WALK_ALL ? std::min<uint32_t>(C, 8) : 1)) << (2 * grow), ops_max_of(j));
+    }
     uint64_t out_bytes(const host::Job &j) const {
         const uint64_t C = al.layouts.layouts[j.layout].ent.size();
-        return (uint64_t)(2 * j.n + 4 * C + 64) * sizeof(OutOp) + 4096;
+        return ops_cap_of(j, 0) * sizeof(OutOp) + (j.walk == host::WALK_ALL ? C : 1) * sizeof(ChainHdr) + 4096;
     }
 
     void run(const std::vector<host::Job> &jobs, std::vector<host::JobResult> &out) override {
@@ -286,6 +300,7 @@ struct CudaBackend : host::Backend {
             }
         }
         size_up();
+        ops_grow.assign(jobs.size(), 0);
         for (size_t k = 0; k < jobs.size(); ++k)
             if (bytes[k] > mem_budget) throw Error(STITCH_ERR_NOMEM, "one read's checkpoints do not fit in device memory");
         const uint64_t n_chunks = (total + cap - 1) / cap;
@@ -297,7 +312,6 @@ struct CudaBackend : host::Backend {
                 if (end > begin && (used + bytes[end] > cap || used >= target || (max_inflight && end - begin >= max_inflight))) break;
                 used += bytes[end]; ++end;
             }
-            struct ScaleGuard { uint32_t &s; ~ScaleGuard() { s = 1; } } guard{ops_scale};   // (also when a retry throws)
             run_chunk(jobs, begin, end, out);
             begin = end;
         }
@@ -344,8 +358,7 @@ struct CudaBackend : host::Backend {
             d.colrec_off = tot.colrec; d.cell_off = tot.cell; d.cksum_off = tot.cksum; d.gcol_off = tot.gcol; d.ops_off = ops_n;
             d.n = j.n; d.layout = j.layout; d.walk = j.walk; d.from_contig = j.from_contig;
             d.max_chains = j.walk == host::WALK_ALL ? C : 1;
-            const uint32_t per_chain = j.n / 2 + 4 * C + 64;
-            d.ops_cap = per_chain * (j.walk == host::WALK_ALL ? std::min<uint32_t>(C, 8) : 1) * ops_scale;
+            d.ops_cap = (uint32_t)ops_cap_of(j, ops_grow[begin + k]);
             d.chain_first = (uint32_t)chains_n;
             d.track_from = tracked ? (j.n > WINDOW ? j.n - WINDOW + 1 : 1) : j.n + 1;
             d.hand_off = tot.cell; d.handsum_off = handsum_n;
@@ -605,13 +618,16 @@ struct CudaBackend : host::Backend {
 
         bool overflow = false;
         for (uint32_t k = 0; k < nj; ++k) {
-            if (h_jobout.p[k].status == WALK_OVERFLOW) overflow = true;
-            else if (h_jobout.p[k].status != WALK_OK)
+            if (h_jobout.p[k].status == WALK_OVERFLOW) {
+                // rare: rerun the chunk with x4 the operation buffer of every read that overflowed; a buffer that already
+                // holds chain_ops_bound per chain cannot have overflowed
+                if (h_jobs.p[k].ops_cap >= ops_max_of(jobs[begin + k])) throw Error(STITCH_ERR_INTERNAL, "operation buffer overflow");
+                ++ops_grow[begin + k];
+                overflow = true;
+            } else if (h_jobout.p[k].status != WALK_OK)
                 throw Error(STITCH_ERR_INTERNAL, "traceback reached a state the reference panics on");
         }
         if (overflow) {
-            if (ops_scale >= 64) throw Error(STITCH_ERR_INTERNAL, "operation buffer overflow");
-            ops_scale *= 4;   // rare: rerun the chunk with larger operation buffers (run() resets the scale after the chunk)
             for (size_t k = begin; k < end; ++k) out[k] = host::JobResult();
             run_chunk(jobs, begin, end, out);
             return;
@@ -711,7 +727,7 @@ struct CudaBackend : host::Backend {
         cudaError_t se = cudaStreamSynchronize(stream);
         if (se != cudaSuccess) throw Error(STITCH_ERR_CUDA, std::string("kernel failed (") + what + "): " + cudaGetErrorString(se));
     }
-    uint32_t ops_scale = 1;
+    std::vector<uint32_t> ops_grow;   // per job of the current run(): x4 growths of its operation buffer (retries)
 };
 
 }  // namespace gpu

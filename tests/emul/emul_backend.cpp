@@ -936,6 +936,16 @@ Backend *stitch_make_backend(Aligner &al, int) { return new EmulBackend(al); }
 }  // namespace host
 }  // namespace stitch
 
+// sizeof of the device structs whose sizes tests/ckplan.py uses to restate the shared-memory layouts of the CUDA kernels
+// (PkColConst: kernels_packed.cuh, not compiled here; same members)
+extern "C" void emul_struct_sizes(uint32_t *out) {
+    using namespace stitch;
+    struct PkColConst { PCol pc; int32_t r0pkey, cr1key; uint8_t yq[PKQ_L + 2]; };
+    const uint32_t s[] = {sizeof(JumpInfo), sizeof(PkRowM), sizeof(PkQuiet), sizeof(ContigEntry), sizeof(PkColConst), sizeof(RowM),
+                          sizeof(XsPart), sizeof(CmPart), sizeof(ICarry)};
+    for (size_t k = 0; k < sizeof(s) / sizeof(s[0]); ++k) out[k] = s[k];
+}
+
 // pk_plan (dp_packed.h) of the scoring the product derives from these options: the length bits of the packed path, 0 = the
 // wide path, -1 = options the product refuses
 extern "C" int32_t emul_pk_plan(const stitch_opts *o, uint32_t n, uint32_t m_max) {

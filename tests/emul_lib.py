@@ -49,8 +49,20 @@ def lib(strip=8):
     e.emul_pk_plan.argtypes = [C.POINTER(StitchOpts), C.c_uint32, C.c_uint32]
     e.emul_path_counters.restype = None
     e.emul_path_counters.argtypes = [C.POINTER(C.c_ulonglong)]
+    e.emul_struct_sizes.restype = None
+    e.emul_struct_sizes.argtypes = [C.POINTER(C.c_uint32)]
     _libs[strip] = e
     return e
+
+
+STRUCT_NAMES = ("JumpInfo", "PkRowM", "PkQuiet", "ContigEntry", "PkColConst", "RowM", "XsPart", "CmPart", "ICarry")
+
+
+def struct_sizes(strip=8):
+    """sizeof of the structs the kernels' shared-memory layouts are carved from: {name: bytes}."""
+    out = (C.c_uint32 * len(STRUCT_NAMES))()
+    lib(strip).emul_struct_sizes(out)
+    return dict(zip(STRUCT_NAMES, out))
 
 
 def pk_plan(opts: StitchOpts, n, m_max, strip=8):
