@@ -35,6 +35,10 @@ extern "C" {
 /* AlignmentMode, LIB/align/aligners/constants.rs:96-108 (Custom is rejected, mod.rs:129). */
 enum { STITCH_MODE_LOCAL = 0, STITCH_MODE_QUERY_LOCAL = 1, STITCH_MODE_TARGET_LOCAL = 2, STITCH_MODE_GLOBAL = 3 };
 
+/* stitch_opts.pre_align_scoring (definitions: stitch_b200/csrc/prealign_core.h).  KMER: the bases covered by exact k-mer
+ * hits in the best band of 2 band_width diagonals.  BANDED: the best local affine-gap alignment inside that band. */
+enum { STITCH_PREALIGN_KMER = 0, STITCH_PREALIGN_BANDED = 1 };
+
 /* AlignmentOperation, LIB/align/aligners/constants.rs:20-29.  Runs of Match/Subst/Del/Ins are
  * run-length encoded: `a` is the run length.  Xclip/Yclip/Yjump: `a` is the length.
  * Xjump: `a` = contig index, `b` = 0-based contig offset the chain continues at. */
@@ -72,7 +76,8 @@ typedef struct stitch_opts {
     /* Pre-alignment contig selection (Options.pre_align .. pre_align_subset_contigs, mod.rs:76-86; align.rs:119-146). */
     uint8_t pre_align;            /* -p: only reads with a pre-alignment score >= pre_align_min_score are aligned   */
     uint8_t pre_align_subset_contigs; /* -x: align such a read to the contig-strands that reached the score only     */
-    uint8_t reserved1[2];
+    uint8_t pre_align_scoring;    /* STITCH_PREALIGN_*: how a contig-strand is scored (default k-mer; 0 = k-mer)   */
+    uint8_t reserved1[1];
     uint32_t kmer_size;           /* -k, default 12                                          */
     uint32_t band_width;          /* -w, default 50                                          */
     int32_t pre_align_min_score;  /* -s, default 100                                         */

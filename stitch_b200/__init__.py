@@ -71,7 +71,7 @@ class Builder:
                    jump_score_same_contig_opposite_strand=None, jump_score_inter_contig=None,
                    double_strand=False, circular=False, circular_slop=20, suboptimal=False,
                    suboptimal_pct=20.0, pre_align=False, pre_align_subset_contigs=True, kmer_size=12, band_width=50,
-                   pre_align_min_score=100)
+                   pre_align_min_score=100, pre_align_scoring="kmer")
 
     def __init__(self, **kw):
         self._v = dict(self._FIELDS)

@@ -4,6 +4,9 @@ import ctypes as C
 MODE_LOCAL, MODE_QUERY_LOCAL, MODE_TARGET_LOCAL, MODE_GLOBAL = 0, 1, 2, 3
 OP_MATCH, OP_SUBST, OP_DEL, OP_INS, OP_XCLIP, OP_YCLIP, OP_XJUMP, OP_YJUMP = range(8)
 
+PREALIGN_KMER, PREALIGN_BANDED = 0, 1
+PREALIGN_SCORING = {"kmer": PREALIGN_KMER, "banded": PREALIGN_BANDED}   # stitch_opts.pre_align_scoring
+
 MODE_NAMES = {
     # AlignmentMode::from_str, fg-stitch-lib/src/align/aligners/constants.rs:121-136
     "local": MODE_LOCAL,
@@ -20,7 +23,8 @@ class StitchOpts(C.Structure):
         ("jump_same", C.c_int32), ("jump_opp", C.c_int32), ("jump_inter", C.c_int32),
         ("double_strand", C.c_uint8), ("circular", C.c_uint8), ("suboptimal", C.c_uint8), ("reserved0", C.c_uint8),
         ("circular_slop", C.c_uint32), ("suboptimal_pct", C.c_float),
-        ("pre_align", C.c_uint8), ("pre_align_subset_contigs", C.c_uint8), ("reserved1", C.c_uint8 * 2),
+        ("pre_align", C.c_uint8), ("pre_align_subset_contigs", C.c_uint8), ("pre_align_scoring", C.c_uint8),
+        ("reserved1", C.c_uint8 * 1),
         ("kmer_size", C.c_uint32), ("band_width", C.c_uint32), ("pre_align_min_score", C.c_int32),
     ]
 
@@ -64,10 +68,15 @@ def make_opts(mode=MODE_LOCAL, match_score=1, mismatch_score=-4, gap_open=-6, ga
               jump_score_same_contig_opposite_strand=None, jump_score_inter_contig=None,
               double_strand=False, circular=False, circular_slop=20, suboptimal=False,
               suboptimal_pct=20.0, pre_align=False, pre_align_subset_contigs=True, kmer_size=12, band_width=50,
-              pre_align_min_score=100) -> StitchOpts:
-    """Options with the reference's defaults (aligners/mod.rs:67-116, 143-152)."""
+              pre_align_min_score=100, pre_align_scoring="kmer") -> StitchOpts:
+    """Options with the reference's defaults (aligners/mod.rs:67-116, 143-152).  `pre_align_scoring`: "kmer" (default)
+    or "banded" (stitch_b200/csrc/prealign_core.h); an int is passed through as it is."""
     if isinstance(mode, str):
         mode = MODE_NAMES[mode.lower()]
+    if isinstance(pre_align_scoring, str):
+        if pre_align_scoring not in PREALIGN_SCORING:
+            raise ValueError(f"pre_align_scoring must be one of {sorted(PREALIGN_SCORING)}, got {pre_align_scoring!r}")
+        pre_align_scoring = PREALIGN_SCORING[pre_align_scoring]
     pick = lambda v: default_jump_score if v is None else v
     return StitchOpts(
         mode=mode, match_score=match_score, mismatch_score=mismatch_score, gap_open=gap_open,
@@ -76,7 +85,7 @@ def make_opts(mode=MODE_LOCAL, match_score=1, mismatch_score=-4, gap_open=-6, ga
         double_strand=int(bool(double_strand)), circular=int(bool(circular)), suboptimal=int(bool(suboptimal)),
         reserved0=0, circular_slop=int(circular_slop), suboptimal_pct=float(suboptimal_pct),
         pre_align=int(bool(pre_align)), pre_align_subset_contigs=int(bool(pre_align_subset_contigs)), kmer_size=int(kmer_size),
-        band_width=int(band_width), pre_align_min_score=int(pre_align_min_score))
+        band_width=int(band_width), pre_align_min_score=int(pre_align_min_score), pre_align_scoring=int(pre_align_scoring))
 
 
 def make_contigs(contigs):

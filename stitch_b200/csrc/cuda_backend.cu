@@ -649,6 +649,8 @@ struct CudaBackend : host::Backend {
     DevBuf<uint32_t> d_koff, d_kpos, d_seqoff, d_slen, d_pcnt, d_pbins, d_poutn, d_prlen;
     DevBuf<uint64_t> d_proff;
     DevBuf<PreHit> d_pout;
+    DevBuf<int32_t> d_pband;
+    bool prealign_scores_banded() const override { return true; }
     void prealign(const std::vector<host::Job> &reads, std::vector<std::vector<PreHit>> &out) override {
         CUDA_CHECK(cudaSetDevice(device));
         out.assign(reads.size(), std::vector<PreHit>());
@@ -677,6 +679,8 @@ struct CudaBackend : host::Backend {
             const uint32_t n_bins = (max_n + c.max_len) / o.band + 2;
             d_proff.reserve(nr); d_prlen.reserve(nr); d_pout.reserve(nr * MAX_STRANDS); d_poutn.reserve(nr);
             d_pcnt.reserve((size_t)grid * c.n_strands); d_pbins.reserve((size_t)grid * PRE_MAX_CAND * n_bins);
+            const uint32_t band_chunks = (2 * o.band + PRE_BAND_CHUNK - 1) / PRE_BAND_CHUNK;   // banded: windows of 2 W diagonals
+            if (o.pre_banded && band_chunks > 1) d_pband.reserve((size_t)grid * (PRE_THREADS / 32) * 2 * band_chunks * PRE_BAND_CHUNK);
             CUDA_CHECK(cudaEventRecord(e0, stream));
             CUDA_CHECK(cudaMemcpyAsync(d_reads.p, h_reads.p, bytes, cudaMemcpyHostToDevice, stream));
             CUDA_CHECK(cudaMemcpyAsync(d_proff.p, offs.data(), nr * 8, cudaMemcpyHostToDevice, stream));
@@ -687,6 +691,8 @@ struct CudaBackend : host::Backend {
             P.n_strands = c.n_strands; P.K = o.kmer; P.W = o.band; P.n_bins = n_bins; P.match = o.sc.match; P.min_score = o.pre_min_score;
             P.reads = d_reads.p; P.read_off = d_proff.p; P.read_len = d_prlen.p; P.n_reads = (uint32_t)nr;
             P.counter = d_counter.p; P.cnt = d_pcnt.p; P.bins = d_pbins.p; P.out = d_pout.p; P.out_n = d_poutn.p;
+            P.banded = o.pre_banded; P.mismatch = o.sc.mismatch; P.gap_open = o.sc.o; P.gap_extend = o.sc.e;
+            P.band_chunks = band_chunks; P.band_rows = o.pre_banded && band_chunks > 1 ? d_pband.p : nullptr;
             prealign_kernel<<<grid, PRE_THREADS, 0, stream>>>(P);
             CUDA_CHECK(cudaGetLastError());
             hout.resize(nr * MAX_STRANDS); hn.resize(nr);

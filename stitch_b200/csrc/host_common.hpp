@@ -41,6 +41,7 @@ struct Opts {
     uint32_t slop = 20;
     float sub_pct = 20.0f;
     bool pre_align = false, pre_subset = true;   // mod.rs:76-86
+    bool pre_banded = false;                     // STITCH_PREALIGN_BANDED (prealign_core.h)
     uint32_t kmer = 12, band = 50;
     int32_t pre_min_score = 100;
 };
@@ -68,6 +69,9 @@ inline Opts make_opts(const stitch_opts &o) {
     p.slop = o.circular_slop; p.sub_pct = o.suboptimal_pct;
     p.pre_align = o.pre_align != 0; p.pre_subset = o.pre_align_subset_contigs != 0;
     p.kmer = o.kmer_size; p.band = o.band_width; p.pre_min_score = o.pre_align_min_score;
+    if (o.pre_align_scoring != STITCH_PREALIGN_KMER && o.pre_align_scoring != STITCH_PREALIGN_BANDED)
+        throw Error(STITCH_ERR_INVALID, "pre-alignment scoring must be 0 (k-mer) or 1 (banded)");
+    p.pre_banded = o.pre_align_scoring == STITCH_PREALIGN_BANDED;
     if (p.pre_align) {
         if (p.kmer < 4 || p.kmer > 31) throw Error(STITCH_ERR_INVALID, "k-mer size must be 4..31");
         if (p.band < 1) throw Error(STITCH_ERR_INVALID, "band width must be positive");
@@ -241,10 +245,68 @@ struct KmerIndex {
     }
 };
 
+// The pre-alignment exactly as prealign_core.h defines it, sequentially, for either scoring (opts.pre_banded): per read the
+// selected contig-strands in ascending order with their scores.  The statement of the definition the backends are checked
+// against; it runs for a backend that does not implement the banded scoring itself (Backend::prealign_scores_banded).
+inline void prealign_sequential(const Opts &o, const Contigs &c, KmerIndex &kindex, const std::vector<Job> &reads,
+                                std::vector<std::vector<PreHit>> &out) {
+    if (kindex.K != o.kmer) kindex.build(c, o.kmer);
+    out.assign(reads.size(), std::vector<PreHit>());
+    const uint32_t K = o.kmer, W = o.band;
+    for (size_t r = 0; r < reads.size(); ++r) {
+        const uint8_t *read = reads[r].read; const uint32_t n = reads[r].n;
+        std::vector<uint32_t> cnt(c.n_strands, 0);
+        std::vector<std::pair<uint32_t, uint32_t>> hits;   // (strand, diagonal + n)
+        for (uint32_t j = 0; j + K <= n; ++j) {
+            uint64_t code;
+            if (!pre_kmer_code(read + j, K, code)) continue;
+            const uint32_t b = pre_bucket(code, K);
+            for (uint32_t e = kindex.off[b]; e < kindex.off[b + 1]; ++e) {
+                const uint32_t p = kindex.pos[e];
+                if (K > PRE_DIRECT_K && !pre_same_kmer(c.blob.data() + p, read + j, K)) continue;
+                const uint32_t s = pre_strand_of(c.seq_off.data(), c.n_strands, p);
+                ++cnt[s]; hits.emplace_back(s, (p - c.seq_off[s]) + n - j);
+            }
+        }
+        uint32_t need = o.pre_banded ? pre_need_banded(o.pre_min_score, o.sc.match, K) : pre_need(o.pre_min_score, o.sc.match, K);
+        std::vector<uint32_t> cand;
+        for (;;) {
+            cand.clear();
+            for (uint32_t s = 0; s < c.n_strands; ++s) if (cnt[s] >= need) cand.push_back(s);
+            if (cand.size() <= PRE_MAX_CAND) break;
+            need *= 2;
+        }
+        const uint32_t n_bins = (n + c.max_len) / W + 2;
+        std::vector<PreHit> kept;
+        for (uint32_t s : cand) {
+            std::vector<uint32_t> bins(n_bins, 0);
+            for (const auto &h : hits) if (h.first == s && h.second / W < n_bins) ++bins[h.second / W];
+            uint32_t best = 0, bstar = 0;   // the lowest bin of the best pair
+            for (uint32_t b = 0; b < n_bins; ++b) {
+                const uint32_t v = bins[b] + (b + 1 < n_bins ? bins[b + 1] : 0u);
+                if (v > best) { best = v; bstar = b; }
+            }
+            const int32_t dlo = (int32_t)(bstar * W) - (int32_t)n, dhi = dlo + 2 * (int32_t)W;
+            const int32_t sc = o.pre_banded ? pre_banded_score(read, n, c.blob.data() + c.seq_off[s], c.len[s], dlo, dhi, o.sc)
+                                            : pre_score_of(o.sc.match, best, K);
+            if (sc >= o.pre_min_score) kept.push_back(PreHit{s, sc});
+        }
+        if (kept.size() > MAX_STRANDS) {
+            std::stable_sort(kept.begin(), kept.end(), [](const PreHit &a, const PreHit &b) { return a.score != b.score ? a.score > b.score : a.strand < b.strand; });
+            kept.resize(MAX_STRANDS);
+            std::sort(kept.begin(), kept.end(), [](const PreHit &a, const PreHit &b) { return a.strand < b.strand; });
+        }
+        out[r] = kept;
+    }
+}
+
 struct Backend {
     virtual ~Backend() {}
     // Pre-alignment (prealign_core.h): per read, the selected contig-strands in ascending order with their scores.
     virtual void prealign(const std::vector<Job> &reads, std::vector<std::vector<PreHit>> &out) = 0;
+    // Whether prealign() implements the banded scoring too (the CUDA backend: kernels_prealign.cuh).  With a backend that
+    // implements only the k-mer scoring (the CPU emulator the tests run), the banded scoring comes from prealign_sequential.
+    virtual bool prealign_scores_banded() const { return false; }
     // `device_reads`: reads already resident on the device (d_bases base pointer + per-job offsets
     // in Job::read interpreted as offsets); only the CUDA backend supports it.
     virtual void run(const std::vector<Job> &jobs, std::vector<JobResult> &out) = 0;
@@ -406,6 +468,13 @@ struct Aligner {
     LayoutCache layouts;
     std::unique_ptr<Backend> backend;
     std::string last_error;
+    KmerIndex seq_kindex;   // prealign_sequential's index (built on first use)
+
+    // The pre-alignment of a batch under opts' scoring (see Backend::prealign_scores_banded).
+    void prealign(const std::vector<Job> &reads, std::vector<std::vector<PreHit>> &hits) {
+        if (opts.pre_banded && !backend->prealign_scores_banded()) prealign_sequential(opts, contigs, seq_kindex, reads, hits);
+        else backend->prealign(reads, hits);
+    }
 
     void init(const stitch_opts &o, const stitch_contig *c, uint32_t n) {
         opts = make_opts(o);
@@ -554,7 +623,7 @@ struct Aligner {
             pj[r].read = q[r].data(); pj[r].n = (uint32_t)q[r].size();
         }
         std::vector<std::vector<PreHit>> hits;
-        backend->prealign(pj, hits);
+        prealign(pj, hits);
         std::fill(words, words + (size_t)n_reads * stride, 0u);
         for (uint32_t r = 0; r < n_reads; ++r) {
             int32_t b = 0;
@@ -583,7 +652,7 @@ struct Aligner {
             std::vector<Job> pj(n_reads);
             for (uint32_t r = 0; r < n_reads; ++r) { pj[r].read = q[r].data(); pj[r].n = (uint32_t)q[r].size(); }
             std::vector<std::vector<PreHit>> hits;
-            backend->prealign(pj, hits);
+            prealign(pj, hits);
             for (uint32_t r = 0; r < n_reads; ++r) {
                 if (prealign_select(hits[r], pre_strands[r], pre_score[r])) has_pre[r] = 1;
                 else dropped[r] = 1;

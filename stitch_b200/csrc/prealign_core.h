@@ -22,8 +22,23 @@
 //   selected     strands with score(s) >= min_score; if more than MAX_STRANDS (256, the per-read limit of the aligner),
 //                the 256 best by (score descending, strand ascending).
 // Everything is a count, so the result does not depend on the order the GPU's atomics happen to run in.
+//
+// That is the k-mer scoring (STITCH_PREALIGN_KMER, the default).  The banded scoring (STITCH_PREALIGN_BANDED) keeps hits,
+// bins and the caps above and changes three things:
+//   candidates   hits(s) >= need_b, need_b = max(1, ceil(need / 2)) (pre_need_banded), doubling as above.  `need` bounds
+//                a k-mer count, not an alignment score: at 5 % substitutions only about 54 % of the 12-mers of a segment
+//                stay intact, so a segment whose alignment reaches min_score can hold far fewer than `need` hits;
+//   window       b* = the bin b with the largest cnt_s[b] + cnt_s[b + 1], the LOWEST b on ties; the window is the
+//                diagonals d = p - j in [b* W - n, (b* + 2) W - n): the two bins chain(s) covers;
+//   score(s)     the best local (Smith-Waterman, floor 0) affine-gap alignment of the read against strand s over the
+//                cells whose diagonal lies in the window and inside both sequences (pre_banded_score): match / mismatch
+//                by byte equality (N matches N, as in the main DP), a gap of length L costs gap_open + L gap_extend,
+//                linear strands (no circular wrap), no clip penalties in any mode.
 #pragma once
 #include "dp_core.h"
+
+#include <algorithm>
+#include <vector>
 
 namespace stitch {
 
@@ -60,6 +75,8 @@ SHD uint32_t pre_need(int32_t min_score, int32_t match, uint32_t K) {
     const int64_t need = bases - (int64_t)K + 1;
     return need < 1 ? 1u : (uint32_t)need;
 }
+// Candidate threshold of the banded scoring (see the top of this file).
+SHD uint32_t pre_need_banded(int32_t min_score, int32_t match, uint32_t K) { return (pre_need(min_score, match, K) + 1) / 2; }
 SHD int32_t pre_score_of(int32_t match, uint32_t chain_hits, uint32_t K) {
     return chain_hits == 0 ? 0 : (int32_t)((int64_t)match * ((int64_t)chain_hits + K - 1));
 }
@@ -68,6 +85,32 @@ SHD uint32_t pre_strand_of(const uint32_t *seq_off, uint32_t n_strands, uint32_t
     uint32_t lo = 0, hi = n_strands;
     while (hi - lo > 1) { const uint32_t mid = (lo + hi) >> 1; if (seq_off[mid] <= p) lo = mid; else hi = mid; }
     return lo;
+}
+
+// score(s) of the banded scoring: a plain sequential Gotoh over the window's diagonals [dlo, dhi) (d = strand position -
+// read position, 0-based).  Row i = read base i - 1, column q = strand base q - 1; H = best local score ending in the cell,
+// E / F = best ending in a gap along the strand / along the read.  A cell outside the window or the sequences counts as
+// H = 0 and opens gaps from there (o + e <= 0, so such a gap never lifts a cell above the floor): the result is the
+// best alignment over the window's cells alone.  The CUDA kernel (kernels_prealign.cuh) computes the same values warp-wide.
+inline int32_t pre_banded_score(const uint8_t *read, uint32_t n, const uint8_t *strand, uint32_t m, int32_t dlo, int32_t dhi,
+                                const Scoring &sc) {
+    const int32_t oe = sc.o + sc.e;
+    std::vector<int32_t> H(m + 1, 0), F(m + 1, oe);   // previous row, by column; never-written cells: outside the window
+    int32_t best = 0;
+    for (int64_t i = 1; i <= (int64_t)n; ++i) {
+        const int64_t q0 = std::max<int64_t>(1, i + dlo), q1 = std::min<int64_t>(m, i + dhi - 1);
+        if (q0 > q1) continue;
+        int32_t diag = H[(size_t)q0 - 1], left = 0, E = oe;   // H(i - 1, q0 - 1); the cell left of q0 is outside
+        for (int64_t q = q0; q <= q1; ++q) {
+            const int32_t s = read[i - 1] == strand[q - 1] ? sc.match : sc.mismatch;
+            const int32_t f = std::max(H[(size_t)q] + oe, F[(size_t)q] + sc.e);
+            const int32_t e = q == q0 ? oe : std::max(left + oe, E + sc.e);
+            const int32_t h = std::max({0, diag + s, e, f});
+            diag = H[(size_t)q]; H[(size_t)q] = h; F[(size_t)q] = f; E = e; left = h;
+            best = std::max(best, h);
+        }
+    }
+    return best;
 }
 
 }  // namespace stitch

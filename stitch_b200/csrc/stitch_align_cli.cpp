@@ -296,7 +296,7 @@ struct Args {
     bool has_same = false, has_opp = false, has_inter = false;
     int jump_same = 0, jump_opp = 0, jump_inter = 0;
     unsigned circular_slop = 20, batch = 2048, kmer = 12, band = 50;
-    int pre_align_min_score = 100;
+    int pre_align_min_score = 100, pre_align_scoring = STITCH_PREALIGN_KMER;
     float filter_secondary_pct = 10.0f, suboptimal_pct = 20.0f;
     std::string command_line;
 };
@@ -332,7 +332,9 @@ void usage() {
         "  -t, --threads <2>                formatter threads (SAM records + BAM encoding; alignment runs on the GPU)\n"
         "  -p, --pre-align                  pre-align reads (k-mer seeding on the GPU) and align only those reaching the score\n"
         "  -k, --k <12>  -w, --w <50>  -s, --pre-align-min-score <100>  -x, --pre-align-subset-contigs <true>\n"
-        "extras: --sam (SAM text instead of BAM)  --gpus <1>  --device <0>  --batch <2048>\n", stderr);
+        "extras: --sam (SAM text instead of BAM)  --gpus <1>  --device <0>  --batch <2048>\n"
+        "  --pre-align-scoring <kmer|banded>  [kmer] score of -p: bases covered by exact k-mer hits in the best band, or\n"
+        "                                   the best local affine-gap alignment inside that band\n", stderr);
 }
 
 Args parse(int argc, char **argv) {
@@ -394,6 +396,12 @@ Args parse(int argc, char **argv) {
         else if (arg == "--gpus") a.gpus = std::stoi(value(arg, inl, has_inl));
         else if (arg == "--device") a.device = std::stoi(value(arg, inl, has_inl));
         else if (arg == "--batch") a.batch = (unsigned)std::stoul(value(arg, inl, has_inl));
+        else if (arg == "--pre-align-scoring") {
+            const std::string v = value(arg, inl, has_inl);
+            if (v == "kmer") a.pre_align_scoring = STITCH_PREALIGN_KMER;
+            else if (v == "banded") a.pre_align_scoring = STITCH_PREALIGN_BANDED;
+            else die("unknown --pre-align-scoring " + v + " (expected kmer or banded)");
+        }
         else die("unknown option " + arg + " (see --help)");
     }
     if (a.reads_fastq.empty() == a.reads_fasta.empty()) die("Must specify exactly one of --reads-fastq or --reads-fasta");
@@ -542,7 +550,7 @@ int main(int argc, char **argv) {
     o.double_strand = a.double_strand; o.circular = a.circular; o.suboptimal = a.suboptimal;
     o.circular_slop = a.circular_slop; o.suboptimal_pct = a.suboptimal_pct;
     o.pre_align = a.pre_align; o.pre_align_subset_contigs = a.pre_align_subset; o.kmer_size = a.kmer; o.band_width = a.band;
-    o.pre_align_min_score = a.pre_align_min_score;
+    o.pre_align_min_score = a.pre_align_min_score; o.pre_align_scoring = (uint8_t)a.pre_align_scoring;
     stitch_sam_opts so{};
     so.soft_clip = a.soft_clip; so.use_eq_and_x = a.use_eq_and_x; so.pick_primary = (uint8_t)a.pick_primary;
     so.filter_secondary = a.filter_secondary; so.filter_secondary_pct = a.filter_secondary_pct;
